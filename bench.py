@@ -2,13 +2,16 @@
 """
 bench.py -- Mpixels/s of the rational-Bloom insert+query hot path on 4K YUV444 inter-frames.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (K1 threshold+count -> exact (k,l,T) -> K2 insert -> K3 query
 -> K3b witness [-> NCCL all-gather of the bit arrays when N > 1]) over one synthetic stream of
 `--frames` 4K YUV444 frames (BASELINE.json configs[2]: 300 frames, p = 0.05, threshold 3.0), i.e.
 frames-1 inter-frame pairs.  `value` is measured with the stream resident in HBM; `e2e` repeats it
 through the host-buffer API call with the H2D / D2H copies inside the timed region.
+
+--dump-outputs DIR writes what the last timed step computed (rank 0's pairs) as DIR/<name>.npy, float32 / float64, under
+DUMP_BUDGET bytes; the inputs are seeded, so two builds run with the same arguments can be compared array for array.
 
 N > 1 is launched by torchrun (one process per GPU); every rank encodes its own stream (weak
 scaling), time = max over ranks of the CUDA-event time, value = all ranks' pixels / that time.
@@ -34,6 +37,7 @@ sys.path.insert(0, ROOT)
 
 METRIC = "Mpixels/s bloom insert+query, 4K YUV444 inter-frame"
 BYTES_PER_PIXEL = 6            # SURVEY.md 8(d): both frames of the pair read once, 2 * 3 * sizeof(uint8)
+DUMP_BUDGET = 48 << 20         # bytes of arrays --dump-outputs writes at most
 
 
 def measured_peaks():
@@ -361,6 +365,31 @@ def kernel_counters(qkernel: str):
         return None
 
 
+def dump_outputs(out_dir, res, packed, seed=2024):
+    """What one encode hands its caller, as .npy files: every pair's PairResult fields and the popcounts of its packed bitmap
+    and witness, plus the packed bytes themselves (one float32 per byte, zero-padded to the longest) for a fixed, seeded sample
+    of pairs -- all of them when they fit in DUMP_BUDGET.  `packed[t]` is st.fetch(t)'s (bitmap, witness, ...)."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"pair_" + f: np.array([getattr(r, f) for r in res], dtype=np.float64)
+           for f in ("n", "ones", "resid", "l", "wlen", "p", "k", "raw")}
+    out["pair_bitmap_popcount"] = np.array([np.bitwise_count(b).sum() for b, *_ in packed], dtype=np.float64)
+    out["pair_witness_popcount"] = np.array([np.bitwise_count(w).sum() for _, w, *_ in packed], dtype=np.float64)
+    row_bytes = 4 * (max(b.size for b, *_ in packed) + max(w.size for _, w, *_ in packed))
+    count = min(len(packed), max(1, DUMP_BUDGET // max(1, row_bytes)))
+    pick = np.sort(np.random.default_rng(seed).choice(len(packed), count, replace=False))
+
+    def padded(rows):
+        a = np.zeros((len(rows), max(1, max(r.size for r in rows))), dtype=np.float32)
+        for i, r in enumerate(rows):
+            a[i, :r.size] = r
+        return a
+    out["sample_pairs"] = pick.astype(np.float64)
+    out["sample_bitmap_bytes"] = padded([packed[t][0] for t in pick])
+    out["sample_witness_bytes"] = padded([packed[t][1] for t in pick])
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -469,6 +498,8 @@ def run_ours(args):
     mism = st.decode_verify()
     roundtrip_ok = not bool(mism.any())
     own_bm = [st.fetch(t, want_mask=False) for t in range(pairs)]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, own_bm)
     # (2) N > 1: every received slot equals the owner's bit array
     gather_check = strong_check = None
     if world > 1 and args.verify_gather:
@@ -672,6 +703,7 @@ def run_ours(args):
 
 
 def main():
+    sys.dont_write_bytecode = True     # the tree may be read-only: the project modules imported below leave no __pycache__ in it
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=5)
@@ -700,8 +732,14 @@ def main():
     ap.add_argument("--ranges", type=int, default=None, help="split each encode into this many pipelined ranges (library default if unset)")
     ap.add_argument("--no-full-frame-check", dest="full_frame_check", action="store_false",
                     help="CPU baseline: skip the full-frame (n = H*W) calibration sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0's pairs; see dump_outputs)")
     ap.set_defaults(verify_gather=True, full_frame_check=True)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
