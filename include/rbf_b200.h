@@ -141,6 +141,16 @@ int rbf_decompress_mask(rbf_ctx* ctx, const uint8_t* bitmap_unpacked, uint64_t l
  *                      -> BloomFilterCompressor.compress (ivc:198-266) on the flattened mask (ivc:924-927). */
 int rbf_stream_create(rbf_ctx* ctx, uint32_t height, uint32_t width, uint32_t channels, uint32_t sample_bytes,
                       uint32_t max_frames, uint32_t max_pairs, rbf_stream** out);
+/* A stream of single images for BloomFilterCompressor.compress_image (bloom_compress.py:348-383): "pair" i of
+ * rbf_stream_encode is image curr_idx[i] (prev_idx must equal curr_idx) and K1 is _binarize_image (bc:67-87) --
+ * gray > threshold with gray = floor(mean of the C samples) for C > 1 (8-bit samples) and the sample itself for C = 1.
+ * C in 1..4 with 1-byte samples, or C = 1 with 2-byte samples; the store holds max_images images (and pairs).
+ * C = 0 (1-byte samples) makes a decode-only stream for rbf_stream_decode: it keeps the per-image bit-array, witness and
+ * mask slots but no image store (upload, encode, apply_diff and median5 return RBF_ERR_STATE; download copies nothing).
+ * Encode / fetch / fetch_batch / decode_verify / stage_ms / k1_only work as for frame streams; "mask_mode",
+ * "gray_mode" and rbf_stream_encode_host are refused with RBF_ERR_STATE. */
+int rbf_stream_create_images(rbf_ctx* ctx, uint32_t height, uint32_t width, uint32_t channels, uint32_t sample_bytes,
+                             uint32_t max_images, rbf_stream** out);
 void rbf_stream_destroy(rbf_stream* s);
 /* per-stream options (no process-global state: two compressors in one process do not interfere):
  *   "k1_only"   1: rbf_stream_encode stops after K1 (mask + counts) -- VideoFrameCompressor._calculate_frame_diff (ivc:784-808);
@@ -170,6 +180,14 @@ int rbf_stream_fetch_batch(rbf_stream* s, uint32_t first, uint32_t count, uint8_
 /* decode the pairs encoded by the last rbf_stream_encode from their own bitmap + witness (ivc:268-307) and
  * compare with the stored masks on the device: mismatches_out[pair] = differing mask words */
 int rbf_stream_decode_verify(rbf_stream* s, uint32_t pairs, uint64_t* mismatches_out);
+/* decode `count` caller-supplied payloads of the stream's n = H*W positions at once (BloomFilterCompressor.decompress,
+ * bc:307-346 / ivc:268-307): payload i is (l[i], wlen[i], k[i]) with its bitmap at bitmaps_packbits + i*bitmap_slot_bytes and its
+ * witness at witness_packbits + i*witness_slot_bytes (np.packbits order).  The decoded mask lands little-bit-order packed at
+ * masks_packed_little + i*mask_slot_bytes; consumed_out[i] = positions that passed the Bloom test (the reference raises
+ * IndexError when that exceeds wlen[i]).  Requires 1 <= l <= n and wlen <= n.  Overwrites the outputs of the last encode. */
+int rbf_stream_decode(rbf_stream* s, uint32_t count, const uint64_t* l, const uint64_t* wlen, const double* k, const rbf_seeds* seeds,
+                      const uint8_t* bitmaps_packbits, uint64_t bitmap_slot_bytes, const uint8_t* witness_packbits,
+                      uint64_t witness_slot_bytes, uint8_t* masks_packed_little, uint64_t mask_slot_bytes, uint64_t* consumed_out);
 int rbf_stream_bitmap_region(rbf_stream* s, void** dptr, uint64_t* stride_bytes);
 /* device time (CUDA events) of the stages of the last rbf_stream_encode, ms.  K1 and K2 are pipelined over ranges of pairs
  * on two streams, so their spans overlap:

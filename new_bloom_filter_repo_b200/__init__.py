@@ -8,6 +8,7 @@ Host code is Python calling hand-written CUDA through a C ABI (include/rbf_b200.
 There is no CPU fallback: importing is cheap, but every entry point needs librbf_b200.so and a B200.
 """
 from . import _cabi
+from . import bloom_compress
 from ._cabi import RbfError
 from .improved_video_compressor import (BloomFilterCompressor, ImprovedVideoCompressor, VideoFrameCompressor)
 from .improved_video_compressor import RationalBloomFilter as IndexRationalBloomFilter

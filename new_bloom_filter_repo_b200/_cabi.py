@@ -46,8 +46,8 @@ EXPORTS = [
     "rbf_filter_create", "rbf_filter_destroy", "rbf_filter_add_indices", "rbf_filter_check_indices",
     "rbf_filter_add_strings", "rbf_filter_check_strings", "rbf_filter_get_bits", "rbf_filter_set_bits",
     "rbf_compress_mask", "rbf_decompress_mask",
-    "rbf_stream_create", "rbf_stream_destroy", "rbf_stream_set_option", "rbf_stream_upload", "rbf_stream_frame_ptr", "rbf_stream_encode",
-    "rbf_stream_encode_host", "rbf_stream_fetch", "rbf_stream_fetch_batch", "rbf_stream_decode_verify", "rbf_stream_bitmap_region", "rbf_stream_stage_ms",
+    "rbf_stream_create", "rbf_stream_create_images", "rbf_stream_destroy", "rbf_stream_set_option", "rbf_stream_upload", "rbf_stream_frame_ptr", "rbf_stream_encode",
+    "rbf_stream_encode_host", "rbf_stream_fetch", "rbf_stream_fetch_batch", "rbf_stream_decode_verify", "rbf_stream_decode", "rbf_stream_bitmap_region", "rbf_stream_stage_ms",
     "rbf_stream_gather_changed", "rbf_stream_apply_diff", "rbf_stream_download", "rbf_median_blur5", "rbf_stream_median5",
     "rbf_nccl_unique_id", "rbf_nccl_init", "rbf_nccl_allgather", "rbf_stream_allgather_bitmaps", "rbf_nccl_destroy",
     "rbf_peer_export", "rbf_peer_open", "rbf_peer_close", "rbf_peer_gather_init", "rbf_peer_gather_half", "rbf_peer_gather_shutdown",
@@ -102,6 +102,7 @@ def _sig(L):
     L.rbf_compress_mask.argtypes = [vp, vp, u64, P(Seeds), dbl, u64, P(MaskInfo), vp, vp]
     L.rbf_decompress_mask.argtypes = [vp, vp, u64, vp, u64, u64, dbl, P(Seeds), vp, P(u64)]
     L.rbf_stream_create.argtypes = [vp, u32, u32, u32, u32, u32, u32, P(vp)]
+    L.rbf_stream_create_images.argtypes = [vp, u32, u32, u32, u32, u32, P(vp)]
     L.rbf_stream_destroy.argtypes = [vp]
     L.rbf_stream_destroy.restype = None
     L.rbf_stream_set_option.argtypes = [vp, C.c_char_p, C.c_int64]
@@ -112,6 +113,7 @@ def _sig(L):
     L.rbf_stream_fetch.argtypes = [vp, u32, vp, vp, vp]
     L.rbf_stream_fetch_batch.argtypes = [vp, u32, u32, vp, u64, vp, u64, vp, u64]
     L.rbf_stream_decode_verify.argtypes = [vp, u32, vp]
+    L.rbf_stream_decode.argtypes = [vp, u32, vp, vp, vp, P(Seeds), vp, u64, vp, u64, vp, u64, vp]
     L.rbf_stream_bitmap_region.argtypes = [vp, P(vp), P(u64)]
     L.rbf_stream_stage_ms.argtypes = [vp, vp]
     L.rbf_stream_gather_changed.argtypes = [vp, u32, vp, u64, vp]

@@ -8,7 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "librbf_b200.so")
 SOURCES = ["rbf_kernels.cu", "rbf_api.cu"]
-HEADERS = ["rbf_hash.cuh", "rbf_kernels.cuh", "rbf_k1_threshold.cuh", "rbf_k2_insert.cuh", "rbf_k3_query.cuh", "rbf_k3b_witness.cuh",
+HEADERS = ["rbf_hash.cuh", "rbf_kernels.cuh", "rbf_k1_threshold.cuh", "rbf_k1_binarize.cuh", "rbf_k2_insert.cuh", "rbf_k3_query.cuh", "rbf_k3b_witness.cuh",
            "rbf_aux_kernels.cuh", os.path.join("..", "..", "include", "rbf_b200.h")]
 
 NVCC_FLAGS = [

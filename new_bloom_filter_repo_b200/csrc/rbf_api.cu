@@ -595,6 +595,7 @@ struct rbf_stream {
     int k1_only = 0;        // stop after K1 (mask + counts): VideoFrameCompressor._calculate_frame_diff
     int mask_mode = 0;      // 0: |dY| > thr (ivc:808); 1: additionally any byte of the pixel differs
     int gray_mode = 0;      // 1: the mask is taken on cv2.COLOR_BGR2GRAY of the pixel (ivc:792-795) instead of on sample 0
+    bool images = false;    // rbf_stream_create_images: pair i is image curr_idx[i], K1 is k_binarize (bloom_compress.py:67-87)
     bool last_k1_only = false;
     size_t bits_hwm = 0, wit_hwm = 0;   // bytes per slot that may hold set bits (see stream_clear_outputs)
     bool wit_dirty_full = false;
@@ -613,11 +614,8 @@ extern "C" void rbf_stream_destroy(rbf_stream* s) {
     delete s;
 }
 
-extern "C" int rbf_stream_create(rbf_ctx* c, uint32_t H, uint32_t W, uint32_t C, uint32_t S, uint32_t max_frames,
-                                 uint32_t max_pairs, rbf_stream** out) {
-    if (!c || !out) return set_err(c, RBF_ERR_INVALID, "rbf_stream_create: NULL");
-    if (!(S == 1 || S == 2) || !(C == 1 || C == 3) || H == 0 || W == 0 || max_frames < 2 || max_pairs < 1)
-        return set_err(c, RBF_ERR_INVALID, "unsupported frame format H=%u W=%u C=%u sample_bytes=%u", H, W, C, S);
+static int stream_alloc(rbf_ctx* c, uint32_t H, uint32_t W, uint32_t C, uint32_t S, uint32_t max_frames, uint32_t max_pairs,
+                        rbf_stream** out) {
     const uint64_t npix = (uint64_t)H * W;
     if (npix > 0xffffff00ULL) return set_err(c, RBF_ERR_INVALID, "frame too large");
     CK(c, cudaSetDevice(c->device));
@@ -663,9 +661,31 @@ extern "C" int rbf_stream_create(rbf_ctx* c, uint32_t H, uint32_t W, uint32_t C,
     return RBF_OK;
 }
 
+extern "C" int rbf_stream_create(rbf_ctx* c, uint32_t H, uint32_t W, uint32_t C, uint32_t S, uint32_t max_frames,
+                                 uint32_t max_pairs, rbf_stream** out) {
+    if (!c || !out) return set_err(c, RBF_ERR_INVALID, "rbf_stream_create: NULL");
+    if (!(S == 1 || S == 2) || !(C == 1 || C == 3) || H == 0 || W == 0 || max_frames < 2 || max_pairs < 1)
+        return set_err(c, RBF_ERR_INVALID, "unsupported frame format H=%u W=%u C=%u sample_bytes=%u", H, W, C, S);
+    return stream_alloc(c, H, W, C, S, max_frames, max_pairs, out);
+}
+
+extern "C" int rbf_stream_create_images(rbf_ctx* c, uint32_t H, uint32_t W, uint32_t C, uint32_t S, uint32_t max_images,
+                                        rbf_stream** out) {
+    if (!c || !out) return set_err(c, RBF_ERR_INVALID, "rbf_stream_create_images: NULL");
+    const bool fmt = (S == 1 && C <= 4) || (S == 2 && C == 1);          // C = 0: decode-only, no image store
+    if (!fmt || H == 0 || W == 0 || max_images < 1)
+        return set_err(c, RBF_ERR_INVALID, "unsupported image format H=%u W=%u C=%u sample_bytes=%u max_images=%u", H, W, C, S, max_images);
+    if (int r = stream_alloc(c, H, W, C, S, max_images, max_images, out)) return r;
+    (*out)->images = true;
+    (*out)->mask_mode = 0;
+    return RBF_OK;
+}
+
 extern "C" int rbf_stream_set_option(rbf_stream* s, const char* key, int64_t v) {
     if (!s || !key) return set_err(s ? s->c : nullptr, RBF_ERR_INVALID, "rbf_stream_set_option: NULL");
     if (!strcmp(key, "k1_only")) { s->k1_only = v ? 1 : 0; return RBF_OK; }
+    if (s->images && v && (!strcmp(key, "mask_mode") || !strcmp(key, "gray_mode")))
+        return set_err(s->c, RBF_ERR_STATE, "%s is a frame-pair option; image streams binarize one image", key);
     if (!strcmp(key, "mask_mode")) { s->mask_mode = v ? 1 : 0; return RBF_OK; }
     if (!strcmp(key, "gray_mode")) {
         if (v && s->C != 3) return set_err(s->c, RBF_ERR_INVALID, "gray_mode needs 3-channel frames");
@@ -678,6 +698,7 @@ extern "C" int rbf_stream_set_option(rbf_stream* s, const char* key, int64_t v) 
 extern "C" int rbf_stream_upload(rbf_stream* s, uint32_t first, uint32_t count, const void* host) {
     if (!s || !host) return set_err(s ? s->c : nullptr, RBF_ERR_INVALID, "rbf_stream_upload: NULL");
     rbf_ctx* c = s->c;
+    if (s->frame_bytes == 0) return set_err(c, RBF_ERR_STATE, "decode-only image stream (0 channels): it has no image store");
     if ((uint64_t)first + count > s->max_frames) return set_err(c, RBF_ERR_INVALID, "frames [%u,%u) exceed store of %u", first, first + count, s->max_frames);
     CK(c, cudaMemcpy2DAsync(s->d_frames + (size_t)first * s->frame_stride, s->frame_stride, host, s->frame_bytes, s->frame_bytes,
                             count, cudaMemcpyHostToDevice, c->st));
@@ -850,7 +871,7 @@ static int stream_encode_pipelined(rbf_stream* s, uint32_t pairs, const uint32_t
                                    double threshold, const rbf_seeds* sd, const double* kov, const uint64_t* lov) {
     rbf_ctx* c = s->c;
     const uint32_t n = (uint32_t)s->npix, ncent = (n + 99u) / 100u;
-    const int thr_int = stream_thr_int(s, threshold);
+    const int thr_int = s->images ? threshold_to_int(threshold) : stream_thr_int(s, threshold);
     uint32_t R = (uint32_t)c->encode_ranges;
     if (R > 8u) R = 8u;
     if (pairs < 8u * R) R = 1u;                          // small jobs: nothing to hide behind
@@ -868,9 +889,13 @@ static int stream_encode_pipelined(rbf_stream* s, uint32_t pairs, const uint32_t
     const int k1_cap = R > 1u ? c->pipe_k1_ctas_per_sm : c->k1_ctas_per_sm;
     for (uint32_t r = 0; r < R; r++) {
         const uint32_t f = lo[r], cnt = lo[r + 1] - lo[r];
-        LAUNCH(c, launch_threshold(s->d_pairs + f, (int)cnt, n, (int)s->C, (int)s->S, thr_int, s->mask_mode, s->gray_mode, s->d_ones + f,
-                                   s->d_resid + f, c->k1_variant, c->sm_count, k1_cap, c->st_k1));
-        if (c->k1_variant == 1 && !s->gray_mode) c->launches++;
+        if (s->images) {
+            LAUNCH(c, launch_binarize(s->d_pairs + f, (int)cnt, n, (int)s->C, (int)s->S, thr_int, s->d_ones + f, c->sm_count, k1_cap, c->st_k1));
+        } else {
+            LAUNCH(c, launch_threshold(s->d_pairs + f, (int)cnt, n, (int)s->C, (int)s->S, thr_int, s->mask_mode, s->gray_mode, s->d_ones + f,
+                                       s->d_resid + f, c->k1_variant, c->sm_count, k1_cap, c->st_k1));
+            if (c->k1_variant == 1 && !s->gray_mode) c->launches++;
+        }
         CK(c, cudaMemcpyAsync(s->h_ones + f, s->d_ones + f, 4 * (size_t)cnt, cudaMemcpyDeviceToHost, c->st_k1));
         CK(c, cudaMemcpyAsync(s->h_resid + f, s->d_resid + f, 4 * (size_t)cnt, cudaMemcpyDeviceToHost, c->st_k1));
         CK(c, cudaEventRecord(c->ev_k1[r], c->st_k1));
@@ -959,6 +984,10 @@ extern "C" int rbf_stream_encode(rbf_stream* s, const uint32_t* prev_idx, const 
     if (!s || !prev_idx || !curr_idx || !sd) return set_err(s ? s->c : nullptr, RBF_ERR_INVALID, "rbf_stream_encode: NULL");
     rbf_ctx* c = s->c;
     if (pairs == 0 || pairs > s->max_pairs) return set_err(c, RBF_ERR_INVALID, "pairs = %u outside [1, %u]", pairs, s->max_pairs);
+    if (s->frame_bytes == 0) return set_err(c, RBF_ERR_STATE, "decode-only image stream (0 channels): nothing to encode");
+    if (s->images)
+        for (uint32_t i = 0; i < pairs; i++)
+            if (prev_idx[i] != curr_idx[i]) return set_err(c, RBF_ERR_INVALID, "image stream: prev_idx[%u] != curr_idx[%u]", i, i);
     CK(c, cudaSetDevice(c->device));
     int rc = stream_encode_pipelined(s, pairs, prev_idx, curr_idx, threshold, sd, kov, lov);
     if (rc) { cudaStreamSynchronize(c->st_k1); cudaStreamSynchronize(c->st); return rc; }
@@ -1033,6 +1062,7 @@ extern "C" int rbf_stream_encode_host(rbf_stream* s, const void* host_frames, ui
     if (!c->st_copy) CK(c, cudaStreamCreateWithFlags(&c->st_copy, cudaStreamNonBlocking));
     if (!c->st_d2h) { CK(c, cudaStreamCreateWithFlags(&c->st_d2h, cudaStreamNonBlocking)); CK(c, cudaEventCreateWithFlags(&c->ev_d2h, cudaEventDisableTiming)); }
     if (s->k1_only) return set_err(c, RBF_ERR_STATE, "rbf_stream_encode_host on a k1_only stream");
+    if (s->images) return set_err(c, RBF_ERR_STATE, "rbf_stream_encode_host codes frame pairs; image streams use rbf_stream_encode");
     // chunks of frames: all H2D copies are queued on the copy stream up front (pinned source), the compute stream
     // encodes a chunk's pairs as soon as its frames have landed, so PCIe transfer and kernels overlap
     const uint32_t CH = c->host_chunk_frames > 1 ? (uint32_t)c->host_chunk_frames : 32u;
@@ -1097,11 +1127,10 @@ extern "C" int rbf_stream_encode_host(rbf_stream* s, const void* host_frames, ui
     return RBF_OK;
 }
 
-extern "C" int rbf_stream_decode_verify(rbf_stream* s, uint32_t pairs, uint64_t* mismatches) {
-    if (!s || !mismatches) return set_err(s ? s->c : nullptr, RBF_ERR_INVALID, "rbf_stream_decode_verify: NULL");
+// Decode slots [0, pairs) of the bit-array / witness regions (packbits order; h_jobs and d_prefix / h_prefix describe the filters)
+// into d_dec (ivc:268-307, bc:307-346); the number of Bloom-test passes of each lands in d_wlen.  Leaves the slots LSB-first.
+static int stream_decode_slots(rbf_stream* s, uint32_t pairs, uint32_t max_l, const uint64_t* wlen) {
     rbf_ctx* c = s->c;
-    if (pairs == 0 || pairs > s->last_pairs) return set_err(c, RBF_ERR_INVALID, "only %u pairs were encoded", s->last_pairs);
-    CK(c, cudaSetDevice(c->device));
     const size_t stride_w = s->mask_stride_w;
     if (!s->d_dec) CK(c, cudaMalloc((void**)&s->d_dec, stride_w * 4 * s->max_pairs));
     CK(c, cudaMemsetAsync(s->d_dec, 0, stride_w * 4 * pairs, c->st));
@@ -1112,14 +1141,26 @@ extern "C" int rbf_stream_decode_verify(rbf_stream* s, uint32_t pairs, uint64_t*
     for (uint32_t i = 0; i < pairs; i++) {
         FrameJob& J = s->h_jobs[i];
         J.out_mask = s->d_dec + (size_t)i * stride_w;
-        J.wlen_in = (uint32_t)s->last_infos[i].wlen;
+        J.wlen_in = (uint32_t)wlen[i];
         J.mask = nullptr;                               // a real decode knows no mask (ivc:286-304)
     }
     CK(c, cudaMemcpyAsync(s->d_jobs, s->h_jobs, sizeof(FrameJob) * pairs, cudaMemcpyHostToDevice, c->st));
     const uint32_t total_cent = s->h_prefix[pairs];
-    LAUNCH(c, launch_query(s->d_jobs, s->d_prefix, (int)pairs, total_cent, s->last_max_l, c->query_variant, c->sm_count, c->query_smem_cap, c->query_warps, c->st));
+    LAUNCH(c, launch_query(s->d_jobs, s->d_prefix, (int)pairs, total_cent, max_l, c->query_variant, c->sm_count, c->query_smem_cap, c->query_warps, c->st));
     LAUNCH(c, launch_expand(s->d_jobs, (int)pairs, (uint32_t)((s->npix + 99) / 100), c->sm_count, s->d_chunkcnt, s->d_wlen, c->st));
     c->launches += 1;
+    return RBF_OK;
+}
+
+extern "C" int rbf_stream_decode_verify(rbf_stream* s, uint32_t pairs, uint64_t* mismatches) {
+    if (!s || !mismatches) return set_err(s ? s->c : nullptr, RBF_ERR_INVALID, "rbf_stream_decode_verify: NULL");
+    rbf_ctx* c = s->c;
+    if (pairs == 0 || pairs > s->last_pairs) return set_err(c, RBF_ERR_INVALID, "only %u pairs were encoded", s->last_pairs);
+    CK(c, cudaSetDevice(c->device));
+    const size_t stride_w = s->mask_stride_w;
+    std::vector<uint64_t> wlen(pairs);
+    for (uint32_t i = 0; i < pairs; i++) wlen[i] = s->last_infos[i].wlen;
+    if (int r = stream_decode_slots(s, pairs, s->last_max_l, wlen.data())) return r;
     void* d_cnt; int rc;
     if ((rc = scratch_get(c, 7, 4 * (size_t)pairs + 4096, &d_cnt))) return rc;
     CK(c, cudaMemsetAsync(d_cnt, 0, 4 * (size_t)pairs, c->st));
@@ -1130,6 +1171,58 @@ extern "C" int rbf_stream_decode_verify(rbf_stream* s, uint32_t pairs, uint64_t*
     CK(c, cudaMemcpyAsync(h.data(), d_cnt, 4 * (size_t)pairs, cudaMemcpyDeviceToHost, c->st));
     CK(c, cudaStreamSynchronize(c->st));
     for (uint32_t i = 0; i < pairs; i++) mismatches[i] = s->last_infos[i].raw ? 0 : h[i];
+    return RBF_OK;
+}
+
+extern "C" int rbf_stream_decode(rbf_stream* s, uint32_t count, const uint64_t* l, const uint64_t* wlen, const double* k,
+                                 const rbf_seeds* sd, const uint8_t* bitmaps, uint64_t bitmap_slot, const uint8_t* witness,
+                                 uint64_t witness_slot, uint8_t* masks_little, uint64_t mask_slot, uint64_t* consumed) {
+    if (!s || !l || !wlen || !k || !sd || !bitmaps || !witness || !masks_little || !consumed)
+        return set_err(s ? s->c : nullptr, RBF_ERR_INVALID, "rbf_stream_decode: NULL");
+    rbf_ctx* c = s->c;
+    if (count == 0 || count > s->max_pairs) return set_err(c, RBF_ERR_INVALID, "count = %u outside [1, %u]", count, s->max_pairs);
+    const uint64_t n = s->npix, mbytes = (n + 7) / 8;
+    const size_t stride = s->mask_stride_w * 4;
+    uint64_t max_l = 0;
+    for (uint32_t i = 0; i < count; i++) {
+        // l > n or wlen > n only come from a corrupt payload; the single-mask decoder (rbf_decompress_mask) takes those
+        if (l[i] == 0 || l[i] > n || wlen[i] > n || !(k[i] >= 0.0) || k[i] > 1e6)
+            return set_err(c, RBF_ERR_INVALID, "image %u: l=%llu wlen=%llu k=%g outside the stream's range (n=%llu)", i,
+                           (unsigned long long)l[i], (unsigned long long)wlen[i], k[i], (unsigned long long)n);
+        if ((l[i] + 7) / 8 > bitmap_slot || (wlen[i] + 7) / 8 > witness_slot)
+            return set_err(c, RBF_ERR_INVALID, "image %u: bitmap / witness larger than its slot", i);
+        if (l[i] > max_l) max_l = l[i];
+    }
+    if (mask_slot < mbytes) return set_err(c, RBF_ERR_INVALID, "mask slot %llu < %llu bytes", (unsigned long long)mask_slot, (unsigned long long)mbytes);
+    CK(c, cudaSetDevice(c->device));
+    if (int r = wait_pack(c)) return r;
+    // the payloads replace the outputs of the last encode: no fetch / decode_verify of it from here on
+    s->last_pairs = 0; s->last_infos.clear(); s->staged = false;
+    const size_t bw = bitmap_slot < stride ? (size_t)bitmap_slot : stride, ww = witness_slot < stride ? (size_t)witness_slot : stride;
+    if (bw > s->bits_hwm) s->bits_hwm = bw;               // the next encode clears what was written here
+    if (ww > s->wit_hwm) s->wit_hwm = ww;
+    CK(c, cudaMemcpy2DAsync(s->d_bits, stride, bitmaps, bitmap_slot, bw, count, cudaMemcpyHostToDevice, c->st));
+    CK(c, cudaMemcpy2DAsync(s->d_wit, stride, witness, witness_slot, ww, count, cudaMemcpyHostToDevice, c->st));
+    c->h2d += (int64_t)(bw + ww) * count;
+    const uint32_t ncent = (uint32_t)((n + 99) / 100);
+    s->h_prefix[0] = 0;
+    for (uint32_t i = 0; i < count; i++) {
+        FrameJob& J = s->h_jobs[i];
+        memset(&J, 0, sizeof J);
+        J.n = (uint32_t)n;
+        job_set_filter(J, l[i], k[i], *sd);
+        J.bits = s->d_bits + (size_t)i * s->mask_stride_w;
+        J.witness = s->d_wit + (size_t)i * s->mask_stride_w;
+        J.pass = s->d_pass + (size_t)i * s->pass_stride_w;
+        s->h_prefix[i + 1] = s->h_prefix[i] + ncent;
+    }
+    CK(c, cudaMemcpyAsync(s->d_prefix, s->h_prefix, 4 * ((size_t)count + 1), cudaMemcpyHostToDevice, c->st));
+    if (int r = stream_decode_slots(s, count, (uint32_t)max_l, wlen)) return r;
+    CK(c, cudaMemcpy2DAsync(masks_little, mask_slot, s->d_dec, stride, mbytes, count, cudaMemcpyDeviceToHost, c->st));
+    CK(c, cudaMemcpyAsync(s->h_wlen, s->d_wlen, 4 * (size_t)count, cudaMemcpyDeviceToHost, c->st));
+    c->d2h += (int64_t)mbytes * count + 4 * (int64_t)count;
+    CK(c, cudaStreamSynchronize(c->st));
+    for (uint32_t i = 0; i < count; i++) consumed[i] = s->h_wlen[i];
     return RBF_OK;
 }
 
@@ -1176,6 +1269,7 @@ extern "C" int rbf_stream_apply_diff(rbf_stream* s, uint32_t base_frame, uint32_
     if (!s || !mask_packed_little || (!values && values_bytes)) return set_err(s ? s->c : nullptr, RBF_ERR_INVALID, "rbf_stream_apply_diff: NULL");
     rbf_ctx* c = s->c;
     if (base_frame >= s->max_frames || out_frame >= s->max_frames) return set_err(c, RBF_ERR_INVALID, "frame index outside the store");
+    if (s->frame_bytes == 0) return set_err(c, RBF_ERR_STATE, "decode-only image stream (0 channels): it has no image store");
     CK(c, cudaSetDevice(c->device));
     const uint64_t pb = (uint64_t)s->C * s->S;
     const size_t mbytes = (size_t)((s->npix + 7) / 8), mwords = s->mask_stride_w;
@@ -1241,6 +1335,7 @@ extern "C" int rbf_median_blur5(rbf_ctx* c, const void* plane_in, uint32_t H, ui
 extern "C" int rbf_stream_median5(rbf_stream* s, uint32_t frame, void* plane_out) {
     if (!s || !plane_out || frame >= s->max_frames) return set_err(s ? s->c : nullptr, RBF_ERR_INVALID, "rbf_stream_median5: bad argument");
     rbf_ctx* c = s->c;
+    if (s->frame_bytes == 0) return set_err(c, RBF_ERR_STATE, "decode-only image stream (0 channels): it has no image store");
     CK(c, cudaSetDevice(c->device));
     const size_t bytes = (size_t)s->npix * s->S;
     void* d_out;

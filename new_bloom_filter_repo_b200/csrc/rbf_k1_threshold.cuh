@@ -300,3 +300,5 @@ __global__ void __launch_bounds__(256) k_threshold_tail(const PairJob* __restric
         if (r) atomicAdd(resid + blockIdx.y, __popc(r));
     }
 }
+
+#include "rbf_k1_binarize.cuh"                         // the single-image K1 shares ldg256_stream

@@ -50,6 +50,9 @@ struct GatherJob {
 cudaError_t launch_threshold(const PairJob* d_pairs, int F, uint32_t npix, int channels, int sample_bytes,
                              int thr_int, int any_mode, int gray_mode, uint32_t* d_ones, uint32_t* d_resid, int variant,
                              int sm_count, int ctas_per_sm, cudaStream_t st);
+// single-image K1 (bloom_compress.py:67-87): PairJob::curr is the image, prev is unused; thr_int = floor of the Python threshold
+cudaError_t launch_binarize(const PairJob* d_images, int F, uint32_t npix, int channels, int sample_bytes, int thr_int,
+                            uint32_t* d_ones, int sm_count, int ctas_per_sm, cudaStream_t st);
 cudaError_t launch_insert(const FrameJob* d_jobs, int F, uint32_t max_centuries, int variant, int sm_count, cudaStream_t st);
 cudaError_t launch_query(const FrameJob* d_jobs, const uint32_t* d_cent_prefix, int F, uint32_t total_centuries,
                          uint32_t max_l_bits, int variant, int sm_count, int smem_bytes_cap, int tile_warps, cudaStream_t st);

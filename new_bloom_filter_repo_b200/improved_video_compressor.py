@@ -99,6 +99,23 @@ class RationalBloomFilter:
         return self._dev.check_strings(strs).astype(bool)
 
 
+def calculate_optimal_params(n: int, p: float) -> Tuple[float, int]:
+    """BloomFilterCompressor._calculate_optimal_params, expression for expression (ivc:161-196; bloom_compress.py:30-64 is the
+    same code)."""
+    if p <= 0.0001:
+        return 0, 0
+    if p >= BloomFilterCompressor.P_STAR:
+        return 0, 0
+    q = 1 - p
+    L = math.log(2)
+    k = math.log2(q * (L ** 2) / p)
+    if math.isnan(k) or k <= 0:
+        return 0, 0
+    gamma = 1 / L
+    l = int(p * n * k * gamma)
+    return max(0.1, k), max(1, l)
+
+
 class BloomFilterCompressor:
     """ivc.BloomFilterCompressor (ivc:140-307)."""
 
@@ -109,18 +126,7 @@ class BloomFilterCompressor:
         self._seeds = seeds
 
     def _calculate_optimal_params(self, n: int, p: float) -> Tuple[float, int]:   # ivc:161-196
-        if p <= 0.0001:
-            return 0, 0
-        if p >= self.P_STAR:
-            return 0, 0
-        q = 1 - p
-        L = math.log(2)
-        k = math.log2(q * (L ** 2) / p)
-        if math.isnan(k) or k <= 0:
-            return 0, 0
-        gamma = 1 / L
-        l = int(p * n * k * gamma)
-        return max(0.1, k), max(1, l)
+        return calculate_optimal_params(n, p)
 
     def compress(self, binary_input: np.ndarray, k_l_override=None):             # ivc:198-266
         """-> (bloom_filter_bitmap, witness, density, input_length, compression_ratio)"""

@@ -29,7 +29,10 @@ class PairResult:
 
 class FrameStream:
     def __init__(self, height: int, width: int, channels: int = 3, dtype=np.uint8, max_frames: int = 2,
-                 max_pairs: Optional[int] = None, k1_only: bool = False, mask_mode: int = 0, gray_mode: bool = False):
+                 max_pairs: Optional[int] = None, k1_only: bool = False, mask_mode: int = 0, gray_mode: bool = False,
+                 images: bool = False):
+        """images=True: a stream of single images (rbf_stream_create_images) -- "pair" i of encode() is image curr_idx[i]
+        (prev_idx == curr_idx) and K1 is _binarize_image (bloom_compress.py:67-87); max_frames images, as many pairs."""
         dt = np.dtype(dtype)
         if dt not in (np.dtype(np.uint8), np.dtype(np.uint16)):
             raise ValueError("frames must be uint8 or uint16")
@@ -38,8 +41,13 @@ class FrameStream:
         self.max_pairs = int(max_pairs if max_pairs is not None else max(1, max_frames - 1))
         self.npix = self.H * self.W
         self._h = C.c_void_p()
-        _cabi.check(_cabi.lib().rbf_stream_create(_cabi.ctx(), self.H, self.W, self.C, dt.itemsize, self.max_frames,
-                                                  self.max_pairs, C.byref(self._h)), _cabi.ctx())
+        if images:
+            self.max_pairs = self.max_frames
+            _cabi.check(_cabi.lib().rbf_stream_create_images(_cabi.ctx(), self.H, self.W, self.C, dt.itemsize, self.max_frames,
+                                                             C.byref(self._h)), _cabi.ctx())
+        else:
+            _cabi.check(_cabi.lib().rbf_stream_create(_cabi.ctx(), self.H, self.W, self.C, dt.itemsize, self.max_frames,
+                                                      self.max_pairs, C.byref(self._h)), _cabi.ctx())
         self._infos = (MaskInfo * self.max_pairs)()
         self.pairs = 0
         self.k1_only = bool(k1_only)
@@ -134,6 +142,28 @@ class FrameStream:
         out = np.zeros(n, dtype=np.uint64)
         _cabi.check(_cabi.lib().rbf_stream_decode_verify(self._h, n, _cabi.ptr(out)), _cabi.ctx())
         return out
+
+    def decode(self, l, wlen, k, bitmaps: np.ndarray, witnesses: np.ndarray, seeds=_cabi.IVC_SEEDS):
+        """Decode caller-supplied payloads of this stream's n positions at once (ivc:268-307, bc:307-346):
+        payload i = (l[i], wlen[i], k[i]) with its packbits bitmap in bitmaps[i] and witness in witnesses[i] (uint8 [count, slot]).
+        -> (masks uint8[count, ceil(n/8)] little bit order, consumed uint64[count] = Bloom-test passes per payload)."""
+        lv = np.ascontiguousarray(np.asarray(l, dtype=np.uint64))
+        wv = np.ascontiguousarray(np.asarray(wlen, dtype=np.uint64))
+        kv = np.ascontiguousarray(np.asarray(k, dtype=np.float64))
+        bm = np.ascontiguousarray(bitmaps, dtype=np.uint8)
+        wt = np.ascontiguousarray(witnesses, dtype=np.uint8)
+        count = lv.size
+        if not (wv.size == kv.size == count == bm.shape[0] == wt.shape[0]):
+            raise ValueError("l, wlen, k, bitmaps and witnesses must describe the same payloads")
+        mslot = (self.npix + 7) // 8
+        masks = np.empty((count, mslot), dtype=np.uint8)
+        consumed = np.zeros(count, dtype=np.uint64)
+        sd = _cabi.seeds_struct(seeds)
+        _cabi.check(_cabi.lib().rbf_stream_decode(self._h, count, _cabi.ptr(lv), _cabi.ptr(wv), _cabi.ptr(kv), C.byref(sd),
+                                                  _cabi.ptr(bm), bm.shape[1], _cabi.ptr(wt), wt.shape[1], _cabi.ptr(masks), mslot,
+                                                  _cabi.ptr(consumed)), _cabi.ctx())
+        self.pairs = 0
+        return masks, consumed
 
     # ------------------------------------------------------------------ N1 / N2 (SURVEY 8f)
     def gather_changed(self, pairs: Optional[int] = None) -> List[np.ndarray]:
